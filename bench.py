@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 30 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # the reference's CPU algorithm on the host cores
+    python bench.py --dump-outputs DIR        # + what the last timed step returned, as DIR/<name>.npy
 
 Workload = BASELINE.json configs[1]: 640x480 synthetic RGB-D stream, ORB 1000 kp/frame, 49 152-word binary
 dictionary, 10 000 signatures.  One "step" = one batch of B independent loop-closure queries (frames); each
@@ -39,6 +40,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 W_WORDS = 49152
 S_SIGS = 10000
@@ -122,6 +124,41 @@ class ClockSampler:
         except OSError:
             pass
         return out
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def step_outputs(words, like, hyp=None, res=None) -> dict:
+    """What a caller of the timed path receives for the frames of one step, one row per frame: word ids, likelihood rows and, where the
+    step verifies, the hypotheses and the verification results.  Integers as float64 (exact), floats at their own precision."""
+    out = {"words": np.asarray(words, np.float64), "likelihood": np.asarray(like, np.float32)}
+    if hyp is not None:
+        out["hypothesis"] = np.asarray(hyp, np.float64)
+        for k in ("ok", "n_matches", "n_inliers", "iterations_run"):
+            out["verify_" + k] = np.array([r[k] for r in res], np.float64)
+        out["verify_rvec"] = np.stack([r["rvec"] for r in res]).astype(np.float64)
+        out["verify_tvec"] = np.stack([r["tvec"] for r in res]).astype(np.float64)
+        out["verify_transform"] = np.stack([r["transform"] for r in res]).astype(np.float32)
+        out["verify_covariance"] = np.stack([r["covariance"] for r in res]).astype(np.float64)
+    return out
+
+
+def dump_outputs(out_dir: str, outputs: dict, prefix: str = "") -> None:
+    """Write `outputs` (step_outputs) as out_dir/<prefix><name>.npy, and the frames they hold as <prefix>frame_index.npy.  Beyond
+    DUMP_LIMIT_BYTES in all (.npy headers included), the same fixed, seeded sample of frames is kept from every array."""
+    n = len(outputs["words"])
+    per_frame = sum(a.nbytes for a in outputs.values()) // max(n, 1) + 8
+    keep = min(n, (DUMP_LIMIT_BYTES - 1024 * (len(outputs) + 1)) // per_frame)
+    if keep == 0:
+        raise SystemExit(f"--dump-outputs: one frame's outputs ({per_frame} bytes) exceed {DUMP_LIMIT_BYTES} bytes")
+    frames = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / f"{prefix}frame_index.npy", frames.astype(np.float64))
+    for name, a in outputs.items():
+        np.save(d / f"{prefix}{name}.npy", a[frames])
+    log(f"wrote the outputs of the last timed step ({keep} of {n} frames) to {d}")
 
 
 def parallelism_text(world_size: int, batch: int) -> str:
@@ -417,6 +454,8 @@ def run_b200(args):
     last_pool = (args.steps - 1) % n_pool
     true_places = places[last_pool * BL:(last_pool + 1) * BL]
     hyp_d, res_d = eng.process_fetch(nf)
+    # captured now: the measurements after the timed loop reuse d_words / d_like
+    outputs = step_outputs(d_words.view(nf, F_FEATS).cpu(), d_like.view(nf, S_SIGS).cpu(), hyp_d, res_d) if args.dump_outputs else None
     def hit_rate(hyp):
         known = true_places >= 0
         return float(np.mean((world.sig_place[np.maximum(hyp, 1) - 1] == true_places)[known] & (hyp[known] > 0))) if known.any() else None
@@ -555,6 +594,8 @@ def run_b200(args):
     e2e_value = B * args.steps / e2e_s
     e2e_hit = hit_rate(np.asarray(hyp_h))
     e2e_verified = float(np.mean([r["ok"] for r in res_h]))
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs, f"rank{rank}_" if world_size > 1 else "")
 
     if rank != 0:
         if world_size > 1:
@@ -872,7 +913,7 @@ def run_reference_c4(args):
 
     for _ in range(min(args.warmup, 1)):
         step()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     total = sum(step() for _ in range(steps))
     value = per_step * steps * (sample / C4_FEATS) / total
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": min(args.warmup, 1),
@@ -952,6 +993,7 @@ def run_c4(args):
     eng.profile_enable(False)
     value = B * args.steps / (dev_ms * 1e-3)
     n_fallback, n_cand, rows_conv = eng.nn_f32_stats(nq)
+    outputs = step_outputs(d_words.view(B, C4_FEATS).cpu(), d_like.view(B, S).cpu()) if args.dump_outputs else None
     like_last = d_like.view(B, S).argmax(1).cpu().numpy()
     last_pool = (args.steps - 1) % n_pool
     hit = float(np.mean(smap.sig_ids[like_last] == smap.sig_ids[places[last_pool * B:(last_pool + 1) * B]]))
@@ -969,6 +1011,8 @@ def run_c4(args):
     e2e_s = time.perf_counter() - t0
     clocks = sampler.stop()
     e2e_value = B * args.steps / e2e_s
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     hbm_peak, peak_src, _ = peaks()
     nn_ms, nn_n = prof["nn"]
@@ -1037,9 +1081,15 @@ def main():
     ap.add_argument("--config", default="c2", choices=["c2", "c4"], help="c2 = BASELINE configs[1] (headline); c4 = configs[3]: float descriptors, 1M words")
     ap.add_argument("--words", type=int, default=0, help="c4: dictionary rows (default 1 000 000)")
     ap.add_argument("--signatures", type=int, default=0, help="c4: signatures in the map (default 100 000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned for its last step as DIR/<name>.npy "
+                                                           "(float32 / float64, at most 64 MB: beyond that a fixed sample of the frames)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         return run_reference(args)
     if args.config == "c4":

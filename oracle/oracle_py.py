@@ -23,12 +23,20 @@ _I = C.c_int
 _F = C.c_float
 
 
+def _reference_readable() -> bool:
+    """Whether the reference sources can be read: a user without access to them still builds and tests, without _ref."""
+    try:
+        return REFERENCE_ROOT.is_dir()
+    except OSError:
+        return False
+
+
 def build(with_ref: bool = True) -> None:
-    """Compile liboracle.so (always) and _ref/libref_flann.so (when /root/reference is present)."""
+    """Compile liboracle.so (always) and _ref/libref_flann.so (when the reference sources are readable)."""
     srcs = [HERE / "oracle.cpp", HERE / "oracle_verify.cpp", HERE / "pnp_math.h"]
     if not LIB.exists() or LIB.stat().st_mtime < max(s.stat().st_mtime for s in srcs):
         subprocess.run(["make", "-C", str(HERE), "liboracle.so"], check=True, capture_output=True)
-    if with_ref and REFERENCE_ROOT.exists() and not REF_LIB.exists():
+    if with_ref and _reference_readable() and not REF_LIB.exists():
         subprocess.run(["make", "-C", str(HERE), "ref"], check=True, capture_output=True)
 
 
@@ -76,11 +84,11 @@ def lib() -> C.CDLL:
 
 
 def ref_lib():
-    """The reference's compiled rtflann, or None when it has not been built (no /root/reference)."""
+    """The reference's compiled rtflann, or None when it has not been built and its sources cannot be read."""
     global _ref
     if _ref is None:
         if not REF_LIB.exists():
-            if REFERENCE_ROOT.exists():
+            if _reference_readable():
                 build(with_ref=True)
             else:
                 return None

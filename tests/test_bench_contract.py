@@ -33,3 +33,34 @@ def test_other_ranks_of_the_reference_arm_exit_quietly():
     p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
                        cwd=ROOT, env=env, capture_output=True, text=True, timeout=120)
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_frames_under_the_limit(tmp_path, monkeypatch):
+    import importlib.util
+
+    import numpy as np
+
+    spec = importlib.util.spec_from_file_location("bench_module", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    rng = np.random.default_rng(0)
+    n = 50
+    res = [{"ok": bool(i % 2), "n_matches": i, "n_inliers": i // 2, "iterations_run": 3 * i, "rvec": rng.random(3), "tvec": rng.random(3),
+            "transform": rng.random((3, 4)).astype(np.float32), "covariance": rng.random((6, 6))} for i in range(n)]
+    out = bench.step_outputs(rng.integers(0, 1 << 20, (n, 1000), dtype=np.int32), rng.random((n, 2000), dtype=np.float32),
+                             rng.integers(0, 100, n, dtype=np.int32), res)
+    bench.dump_outputs(str(tmp_path / "all"), out)
+    assert np.array_equal(np.load(tmp_path / "all" / "frame_index.npy"), np.arange(n))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 300_000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), out)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == sorted(["frame_index.npy"] + [k + ".npy" for k in out])
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 300_000
+    frames = np.load(tmp_path / "a" / "frame_index.npy").astype(np.int64)
+    assert 0 < len(frames) < n and np.all(np.diff(frames) > 0)
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)
+        if f != "frame_index.npy":
+            assert np.array_equal(a, out[f[:-4]][frames])

@@ -1,5 +1,6 @@
 """Parity at the sizes BASELINE.json's configs name (VERDICT r1, item 1) — every check goes through the C ABI and compares with
-the CPU oracle (rtflann-pinned restatement) or with the reference's own compiled rtflann / cv2 where that is the reference:
+the CPU oracle (rtflann-pinned restatement) or with the reference's own compiled rtflann (its answers stored in
+tests/golden/rtflann_knn2.npz) / cv2 where that is the reference:
 
   C1  the reference's own data/samples images (tests/golden/samples_c1.npz): CUDA ORB vs cv::ORB bit for bit on REAL images, then
       the incremental dictionary + raw likelihood of every frame vs the oracle, and the loop-closure recall against samples_GT.bmp
@@ -14,6 +15,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
+from golden_util import rtflann_knn2
 from oracle import feature2d_py as f2d
 from oracle import oracle_py as orc
 from rtabmap_b200 import Engine, synth
@@ -164,13 +166,34 @@ def test_c2_full_size_localisation_batch_of_synthetic_queries(c2_world):
 
 
 # --------------------------------------------------------------------------------------- C3 ---
+C3_W0 = 261000
+C3_K4 = (910.0, 910.0, 640.0, 360.0)
+
+
+def c3_stream():
+    """The initial vocabulary and the 720p frames of test_c3, and the generator that then draws its queries."""
+    rng = np.random.default_rng(12)
+    vocab = synth.make_binary_vocabulary(C3_W0, 32, 5)
+    n_frames = 8
+    imgs = np.stack([synth.make_image(720, 1280, 300 + (k % 5), n_rects=3000) for k in range(n_frames)])
+    for k in range(n_frames):  # later frames re-observe earlier ones with noise: their words must be found among the NEW rows
+        if k >= 5:
+            imgs[k] = np.clip(imgs[k - 5].astype(np.int16) + rng.integers(-3, 4, imgs[k].shape), 0, 255).astype(np.uint8)
+    deps = np.stack([synth.make_depth(720, 1280, 400 + k) for k in range(n_frames)])
+    return vocab, imgs, deps, rng
+
+
+def c3_queries(vocab, frame2_desc, rng):
+    """Noisy copies of initial words and of words the stream created (frame 2's descriptors)."""
+    return synth.flip_bits(np.concatenate([vocab[rng.integers(0, C3_W0, 100)], frame2_desc[:100]]), 0.05, rng)
+
+
 def test_c3_mapping_stream_720p_grows_past_262144_words():
     """configs[2]: 1280x720 frames in mapping mode.  The dictionary starts at 261 000 words (as after a long run / a database load)
     and every frame adds its unmatched descriptors, so the stream crosses 262 144 rows — where the reference's BF strategies stop
     (VWDictionary.cpp:576-583) and only the FLANN-linear order (the rtflann-pinned oracle) is defined."""
-    rng = np.random.default_rng(12)
-    W0 = 261000
-    vocab = synth.make_binary_vocabulary(W0, 32, 5)
+    W0 = C3_W0
+    vocab, imgs, deps, rng = c3_stream()
     ids = np.arange(1, W0 + 1, dtype=np.int32)
     eng = Engine(max_words=300000, max_queries=1000)
     o = orc.OracleDictionary(0, 32, True, 0.8, True)
@@ -178,14 +201,9 @@ def test_c3_mapping_stream_720p_grows_past_262144_words():
         d.add_words(ids, vocab)
         d.last_word_id = W0
         d.update()
-    K4 = (910.0, 910.0, 640.0, 360.0)
+    K4 = C3_K4
     op = Engine.orb_params(K4, n_features=1000)
-    n_frames = 8
-    imgs = np.stack([synth.make_image(720, 1280, 300 + (k % 5), n_rects=3000) for k in range(n_frames)])
-    for k in range(n_frames):  # later frames re-observe earlier ones with noise: their words must be found among the NEW rows
-        if k >= 5:
-            imgs[k] = np.clip(imgs[k - 5].astype(np.int16) + rng.integers(-3, 4, imgs[k].shape), 0, 255).astype(np.uint8)
-    deps = np.stack([synth.make_depth(720, 1280, 400 + k) for k in range(n_frames)])
+    n_frames = len(imgs)
     feats = eng.orb_detect_describe(imgs, deps, op)
     crossed = False
     for t in range(n_frames):
@@ -205,25 +223,22 @@ def test_c3_mapping_stream_720p_grows_past_262144_words():
     # the re-observed frames found words created by this stream (ids above the initial vocabulary)
     assert (g > W0).sum() > 100
     # exact 2-NN over the grown dictionary against the reference's own compiled rtflann
-    q = synth.flip_bits(np.concatenate([vocab[rng.integers(0, W0, 100)], feats[2][1][:100]]), 0.05, rng)
+    q = c3_queries(vocab, feats[2][1], rng)
     gi, gv = eng.get_indexed()
-    r_idx, r_dist = orc.ref_knn2(gv, q)
+    r_idx, r_dist = rtflann_knn2("c3_grown_dictionary", gv, q)
     i1, d1, i2, d2 = eng.knn2(q)
     assert np.array_equal(i1, gi[r_idx[:, 0]]) and np.array_equal(i2, gi[r_idx[:, 1]])
     assert np.array_equal(d1, r_dist[:, 0].astype(np.float32)) and np.array_equal(d2, r_dist[:, 1].astype(np.float32))
 
 
 # --------------------------------------------------------------------------------------- C4 ---
-def test_c4_float_quantiser_over_a_million_rows():
-    """configs[3] size: SURF-like 64-D float descriptors against 1 100 000 dictionary rows (beyond 2^20): exact squared-L2 2-NN ids and
-    distances bit for bit against the reference's compiled rtflann (oracle/_ref), then the NNDR / new-word pass against the oracle."""
-    W = 1_100_000
+C4_W = 1_100_000
+
+
+def c4_problem():
+    """The dictionary rows of test_c4, the rows its queries start from, and the queries."""
+    W = C4_W
     vocab = synth.make_float_vocabulary(W, 64, 21)
-    ids = np.arange(1, W + 1, dtype=np.int32)
-    eng = Engine(desc_type=1, desc_dim=64, max_words=W + 4096, max_queries=1000)
-    eng.add_words(ids, vocab)
-    eng.last_word_id = W
-    eng.update()
     rng = np.random.default_rng(22)
     nq = 96
     src = rng.integers(0, W, nq)
@@ -231,9 +246,21 @@ def test_c4_float_quantiser_over_a_million_rows():
     q = vocab[src] + rng.normal(0, 0.02, (nq, 64)).astype(np.float32)
     q[-16:] = synth.make_float_vocabulary(16, 64, 99)  # unrelated descriptors: NNDR rejects, new words
     q[-8:-4] = q[-16:-12] + np.float32(1e-3)            # near copies of new descriptors inside the frame
-    q = np.ascontiguousarray(q, np.float32)
+    return vocab, src, np.ascontiguousarray(q, np.float32)
+
+
+def test_c4_float_quantiser_over_a_million_rows():
+    """configs[3] size: SURF-like 64-D float descriptors against 1 100 000 dictionary rows (beyond 2^20): exact squared-L2 2-NN ids and
+    distances bit for bit against the reference's compiled rtflann (its stored answer), then the NNDR / new-word pass against the oracle."""
+    W = C4_W
+    vocab, src, q = c4_problem()
+    ids = np.arange(1, W + 1, dtype=np.int32)
+    eng = Engine(desc_type=1, desc_dim=64, max_words=W + 4096, max_queries=1000)
+    eng.add_words(ids, vocab)
+    eng.last_word_id = W
+    eng.update()
     i1, d1, i2, d2 = eng.knn2(q)
-    r_idx, r_dist = orc.ref_knn2(vocab, q)
+    r_idx, r_dist = rtflann_knn2("c4_million_rows", vocab, q)
     assert np.array_equal(i1, ids[r_idx[:, 0]]) and np.array_equal(i2, ids[r_idx[:, 1]])
     assert np.array_equal(d1, r_dist[:, 0]) and np.array_equal(d2, r_dist[:, 1])
     assert (i1[:8] == ids[src[:8]]).all()

@@ -1,15 +1,18 @@
-"""Pin the restated linear 2-NN scan (oracle/oracle.cpp) against the REFERENCE'S OWN rtflann,
-compiled from /root/reference by oracle/Makefile into oracle/_ref/libref_flann.so.
+"""Pin the restated linear 2-NN scan (oracle/oracle.cpp) against the REFERENCE'S OWN rtflann: the answers of its LinearIndex,
+compiled from the reference sources by oracle/Makefile, are stored in tests/golden/rtflann_knn2.npz (make_rtflann_golden.py).
 Covers Hamming (ORB) and squared-L2 (SURF) incl. exact ties and fewer than two rows."""
 import numpy as np
 import pytest
 
+from golden_util import rtflann_knn2
 from oracle import oracle_py as orc
 
-pytestmark = pytest.mark.skipif(orc.ref_lib() is None, reason="oracle/_ref not built (no /root/reference)")
+HAMMING_CASES = [(1, 32), (2, 32), (3, 32), (777, 32), (4096, 32), (1000, 16), (500, 64)]
+L2_CASES = [(2, 64), (1500, 64), (800, 128)]
+KINDS = ["hamming", "l2"]
 
 
-@pytest.mark.parametrize("rows,dim", [(1, 32), (2, 32), (3, 32), (777, 32), (4096, 32), (1000, 16), (500, 64)])
+@pytest.mark.parametrize("rows,dim", HAMMING_CASES)
 def test_hamming_matches_rtflann(rows, dim):
     rng = np.random.default_rng(rows * 7 + dim)
     data = rng.integers(0, 256, (rows, dim), dtype=np.uint8)
@@ -20,14 +23,14 @@ def test_hamming_matches_rtflann(rows, dim):
         q[0] = data[1]
         q[1] = data[rows - 1]
         q[2] = np.bitwise_xor(data[3], 1)
-    i_ref, d_ref = orc.ref_knn2(data, q)
+    i_ref, d_ref = rtflann_knn2(f"hamming_{rows}x{dim}", data, q)
     i_orc, d_orc = orc.knn2_raw(data, q)
     assert np.array_equal(i_ref, i_orc)
     valid = i_ref >= 0
     assert np.array_equal(d_ref[valid], d_orc[valid])
 
 
-@pytest.mark.parametrize("rows,dim", [(2, 64), (1500, 64), (800, 128)])
+@pytest.mark.parametrize("rows,dim", L2_CASES)
 def test_l2_matches_rtflann_bit_exact(rows, dim):
     rng = np.random.default_rng(rows + dim)
     data = rng.standard_normal((rows, dim)).astype(np.float32)
@@ -36,7 +39,7 @@ def test_l2_matches_rtflann_bit_exact(rows, dim):
     if rows > 10:
         data[7] = data[2]
         q[0] = data[2]
-    i_ref, d_ref = orc.ref_knn2(data, q)
+    i_ref, d_ref = rtflann_knn2(f"l2_{rows}x{dim}", data, q)
     i_orc, d_orc = orc.knn2_raw(data, q)
     assert np.array_equal(i_ref, i_orc)
     # same float summation order as rtflann::L2 (dist.h:158-166): identical bits
@@ -44,16 +47,16 @@ def test_l2_matches_rtflann_bit_exact(rows, dim):
 
 
 # ---- the quantiser loop, replayed on the reference's own primitives ---------------------------------------------------
-def _replay_add_new_words(index_ids, index_desc, frame, nndr, last_id, incremental=True, cmp_new=True):
+def _replay_add_new_words(name, index_ids, index_desc, frame, nndr, last_id, incremental=True, cmp_new=True):
     """VWDictionary::addNewWords "Process results" loop (VWDictionary.cpp:1088-1219) written a second time, independently of
-    oracle/oracle.cpp, on the primitives the reference itself calls: its own rtflann LinearIndex (compiled into oracle/_ref)
+    oracle/oracle.cpp, on the primitives the reference itself calls: its own rtflann LinearIndex (its stored answer `name`)
     for the index search and cv::BFMatcher::knnMatch (OpenCV, the installed cv2) for the words created by the same frame.
     fullResults is a std::multimap<float,int>: a stable sort by distance of the insertion sequence."""
     import cv2
 
     binary = frame.dtype == np.uint8
     bf = cv2.BFMatcher(cv2.NORM_HAMMING if binary else cv2.NORM_L2SQR)
-    idx_all, dist_all = (orc.ref_knn2(index_desc, frame) if len(index_desc) else (None, None))
+    idx_all, dist_all = (rtflann_knn2(name, index_desc, frame) if len(index_desc) else (None, None))
     new_desc, new_ids, out = [], [], []
     for i in range(len(frame)):
         full = []
@@ -80,7 +83,7 @@ def _replay_add_new_words(index_ids, index_desc, frame, nndr, last_id, increment
     return np.array(out, np.int32), last_id
 
 
-@pytest.mark.parametrize("kind", ["hamming", "l2"])
+@pytest.mark.parametrize("kind", KINDS)
 def test_quantiser_loop_against_reference_primitives(kind):
     """Pins the NNDR / new-word loop of the oracle (the part of the quantiser the reference has no golden vector for) to an
     independent replay that gets every distance from the reference's rtflann and from cv::BFMatcher."""
@@ -112,7 +115,7 @@ def test_quantiser_loop_against_reference_primitives(kind):
     for t in range(1, 5):
         fresh = rng.integers(0, 256, (120, 32), dtype=np.uint8) if kind == "hamming" else near(rng.standard_normal((120, 64)).astype(np.float32), 0)
         frame = np.concatenate([near(vocab[rng.integers(0, 1200, 50)], 6), fresh, near(fresh[:40], 4), fresh[5:8]])
-        want, last = _replay_add_new_words(index_ids, index_desc, frame, 0.8, last)
+        want, last = _replay_add_new_words(f"quantiser_{kind}_frame{t}", index_ids, index_desc, frame, 0.8, last)
         got = o.add_new_words(frame, t)
         assert np.array_equal(got, want), f"{kind} frame {t}"
         assert o.last_word_id == last
@@ -124,7 +127,7 @@ def test_quantiser_loop_against_reference_primitives(kind):
         o.update()
 
 
-@pytest.mark.parametrize("kind", ["hamming", "l2"])
+@pytest.mark.parametrize("kind", KINDS)
 def test_find_nn_against_reference_primitives(kind):
     """VWDictionary::findNN (VWDictionary.cpp:1273-1552): index hits from the reference's rtflann, hits among the words that are
     not indexed yet from cv::BFMatcher::knnMatch, multimap order, NNDR — replayed independently and compared with the oracle."""
@@ -149,7 +152,7 @@ def test_find_nn_against_reference_primitives(kind):
     o.update()
     o.add_words(pend_ids, pend)            # not indexed: no update()
     o.last_word_id = 2060
-    idx, dist = orc.ref_knn2(vocab, q)
+    idx, dist = rtflann_knn2(f"find_nn_{kind}", vocab, q)
     mni = bf.knnMatch(q, pend, k=2)
     want = np.zeros(len(q), np.int32)
     for i in range(len(q)):
