@@ -128,6 +128,30 @@ int lcd_orb_overflow(lcd_engine * e);
  * threshold >= 19), 4 = vectorised gray / mask preparation (rows a multiple of 8 pixels, even height).  0 = the general kernels. */
 int lcd_orb_last_path(const lcd_engine * e);
 
+/* ---- detector choice: Kp/DetectorStrategy ------------------------------------------
+ * Engine state, like the reference's Feature2D::create (Features2d.cpp:611-700): every entry point that detects
+ * (lcd_orb_detect_describe[_dev], lcd_process_frames*, lcd_map_detect_async, lcd_shard_process_frames_dev) uses the
+ * detector last set here; an engine that never calls lcd_set_detector detects with ORB.
+ * Under LCD_DETECTOR_GFTT_ORB (GFTT/ORB, the reference's default Kp/DetectorStrategy and Vis/FeatureType): corners of
+ * cv::GFTTDetector(maxCorners = n_features, quality_level, min_distance, block_size) inside the depth mask, described by
+ * cv::ORB::compute (corners within ORB/EdgeThreshold of the border are dropped, the rest keep their order; descriptors on
+ * pyramid level 0 with angle -1), then the 3-D lifting of the ORB path.  Of lcd_orb_params, n_features, edge_threshold,
+ * patch_size (31), the depth fields and the camera apply; n_levels, scale_factor and fast_threshold are ignored, and
+ * the image size needs no power-of-two divisibility.  More than 65 536 candidate corners (local maxima above the quality
+ * threshold) in a frame is LCD_ERR_CAPACITY / lcd_orb_overflow, as for the FAST lists. */
+#define LCD_DETECTOR_ORB 2       /* Kp/DetectorStrategy=2, the default of every engine */
+#define LCD_DETECTOR_GFTT_ORB 8  /* Kp/DetectorStrategy=8: cv::GFTTDetector + cv::ORB::compute */
+typedef struct lcd_gftt_params {
+	double quality_level; /* GFTT/QualityLevel (0.001), > 0              */
+	double min_distance;  /* GFTT/MinDistance (7), >= 0                  */
+	int block_size;       /* GFTT/BlockSize (3): 3, 5 or 7               */
+	int use_harris;       /* GFTT/UseHarrisDetector: must be 0           */
+	double k;             /* GFTT/K (0.04): unused while use_harris is 0 */
+} lcd_gftt_params;
+/* strategy LCD_DETECTOR_ORB (gftt may be NULL) or LCD_DETECTOR_GFTT_ORB (gftt required); LCD_ERR_INVALID for anything
+ * else, including the Harris score. */
+int lcd_set_detector(lcd_engine * e, int strategy, const lcd_gftt_params * gftt);
+
 /* ---- dictionary: VWDictionary ------------------------------------------------ */
 /* replaces: VWDictionary::addWord (VWDictionary.cpp:1554-1580) for n words whose ids
  * the caller chose (DB load, LTM reactivation).  Words become "not indexed" until
@@ -491,7 +515,7 @@ int lcd_shard_process_frames_dev(lcd_engine * e, int n_frames, const uint8_t * d
 /* ---- measurement hooks ---------------------------------------------------------------
  * Optional per-kernel timing with CUDA events recorded on the launching stream around
  * every launch of kernel class `which` (0 = dictionary NN, 1 = resolve, 2 = score, 3 = pair
- * matching, 4 = PnP RANSAC, 5 = all ORB kernels).
+ * matching, 4 = PnP RANSAC, 5 = all detect kernels: ORB or GFTT/ORB).
  * lcd_profile_read synchronises, returns the summed device time and the launch count
  * since the last reset. */
 #define LCD_PROF_NN 0
@@ -506,7 +530,7 @@ int lcd_profile_reset(lcd_engine * e);
 
 /* copy an internal ORB buffer of the last lcd_orb_* call back to the host (diagnostics / tests):
  * which = 0 gray pyramid, 1 mask pyramid, 2 blurred pyramid, 3 FAST candidate keys, 4 candidate counts,
- * 5 keypoints per level counts, 6 FAST score pyramid.  Returns the number of bytes copied (<= cap_bytes) or <0. */
+ * 5 keypoints per level counts, 6 FAST score pyramid, 10 GFTT minimum-eigenvalue map (float [n_frames][h][w]).  Returns the number of bytes copied (<= cap_bytes) or <0. */
 long long lcd_debug_orb_buffer(lcd_engine * e, int which, void * out, long long cap_bytes);
 
 /* engine stream (cudaStream_t as void*) and a full device sync, for harnesses */

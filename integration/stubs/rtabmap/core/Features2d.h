@@ -7,7 +7,7 @@ namespace rtabmap {
 class Feature2D
 {
 public:
-	enum Type { kFeatureUndef = -1, kFeatureSurf = 0, kFeatureSift = 1, kFeatureOrb = 2 };             // :117-134
+	enum Type { kFeatureUndef = -1, kFeatureSurf = 0, kFeatureSift = 1, kFeatureOrb = 2, kFeatureGfttOrb = 8 };             // :117-134
 	virtual ~Feature2D() {}                                                                             // :222
 	int getMaxFeatures() const { return maxFeatures_; }                                                 // :214
 	float getMinDepth() const { return _minDepth; }                                                     // :216

@@ -10,6 +10,7 @@ class Parameters
 public:
 	static bool parse(const ParametersMap & p, const std::string & key, int & v) { auto i = p.find(key); if (i == p.end()) return false; v = std::atoi(i->second.c_str()); return true; }
 	static bool parse(const ParametersMap & p, const std::string & key, float & v) { auto i = p.find(key); if (i == p.end()) return false; v = static_cast<float>(std::atof(i->second.c_str())); return true; }
+	static bool parse(const ParametersMap & p, const std::string & key, double & v) { auto i = p.find(key); if (i == p.end()) return false; v = std::atof(i->second.c_str()); return true; }
 	static bool parse(const ParametersMap & p, const std::string & key, bool & v) { auto i = p.find(key); if (i == p.end()) return false; v = i->second == "true" || i->second == "1"; return true; }
 };
 } // namespace rtabmap

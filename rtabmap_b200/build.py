@@ -16,7 +16,7 @@ ROOT = Path(__file__).resolve().parent
 CSRC = ROOT / "csrc"
 LIB = ROOT / "lib" / "liblcd_b200.so"
 SOURCES = ["engine.cu"]
-HEADERS = ["common.cuh", "nn_hamming.cuh", "nn_tensor.cuh", "l2_path.cuh", "nn_tensor_f32.cuh", "resolve.cuh", "score.cuh", "bayes.cuh", "verify.cuh", "match_bf.cuh", "pnp_device.cuh", "orb.cuh", "orb_pattern.h", "../../include/lcd_b200.h"]
+HEADERS = ["common.cuh", "nn_hamming.cuh", "nn_tensor.cuh", "l2_path.cuh", "nn_tensor_f32.cuh", "resolve.cuh", "score.cuh", "bayes.cuh", "verify.cuh", "match_bf.cuh", "pnp_device.cuh", "orb.cuh", "gftt.cuh", "orb_pattern.h", "../../include/lcd_b200.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -54,6 +54,17 @@ class OrbParams(C.Structure):
     ]
 
 
+class GfttParams(C.Structure):
+    """lcd_gftt_params (GFTT/* parameters of the reference, corelib/include/rtabmap/core/Parameters.h:313-317)."""
+    _fields_ = [
+        ("quality_level", C.c_double), ("min_distance", C.c_double), ("block_size", C.c_int), ("use_harris", C.c_int), ("k", C.c_double),
+    ]
+
+
+LCD_DETECTOR_ORB = 2
+LCD_DETECTOR_GFTT_ORB = 8
+
+
 class VerifyParams(C.Structure):
     """lcd_verify_params (Vis/* parameters of the reference, corelib/include/rtabmap/core/Parameters.h:713-754)."""
     _fields_ = [
@@ -112,6 +123,7 @@ SIGNATURES = {
     "lcd_orb_detect_describe_dev": (_I, [_P, _I, _P, _I, _I, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     "lcd_orb_overflow": (_I, [_P]),
     "lcd_orb_last_path": (_I, [_P]),
+    "lcd_set_detector": (_I, [_P, _I, _P]),
     "lcd_dict_add_words": (_I, [_P, _P, _P, _I]),
     "lcd_dict_remove_words": (_I, [_P, _P, _I]),
     "lcd_dict_update": (_I, [_P]),
@@ -288,6 +300,14 @@ class Engine:
                    patch_size=31, min_depth=0.0, max_depth=0.0, depth_as_mask=True):
         return OrbParams(n_features, n_levels, scale_factor, edge_threshold, fast_threshold, patch_size, min_depth, max_depth, int(depth_as_mask),
                          *[float(k) for k in K4])
+
+    @staticmethod
+    def gftt_params(quality_level=0.001, min_distance=7.0, block_size=3, use_harris=False, k=0.04):
+        return GfttParams(float(quality_level), float(min_distance), int(block_size), int(use_harris), float(k))
+
+    def set_detector(self, strategy: int, gftt: "GfttParams" = None):
+        """Kp/DetectorStrategy of every later detection: LCD_DETECTOR_ORB (2) or LCD_DETECTOR_GFTT_ORB (8, needs ``gftt``)."""
+        self._check(self._lib.lcd_set_detector(self._h, int(strategy), C.byref(gftt) if gftt is not None else None))
 
     def orb_detect_describe(self, images, depth, params: "OrbParams", cap: int = 0):
         """images [n,h,w] (gray) or [n,h,w,3] (BGR) uint8; depth [n,h,w] uint16 (mm) / float32 (m) / None.

@@ -21,6 +21,7 @@
 #include "verify.cuh"
 #include "match_bf.cuh"
 #include "orb.cuh"
+#include "gftt.cuh"
 
 #include <cuda.h>
 #include <dlfcn.h>
@@ -327,6 +328,14 @@ struct lcd_engine
 	float gauss_sigma_loaded = -1.f;
 	int orb_tma_used = 0; // the last FAST launch staged its tiles through a tensor map
 	int orb_path = 0;     // lcd_orb_last_path flags of the last detection
+	// detector choice (lcd_set_detector) and the GFTT/ORB workspace
+	int detector = LCD_DETECTOR_ORB;
+	lcd_gftt_params gftt{0.001, 7.0, 3, 0, 0.04};
+	DevBuf<float> g_eig;
+	DevBuf<uint32_t> g_max, g_occ;
+	DevBuf<unsigned long long> g_cand;
+	DevBuf<int> g_cand_count;
+	DevBuf<double> g_rowsum;
 	DevBuf<float> d_uv;
 
 	// measurement hooks (lcd_profile_*)
@@ -2030,6 +2039,124 @@ static int orb_geometry(lcd_engine * e, int width, int height, const lcd_orb_par
 	return LCD_OK;
 }
 
+// GFTT/ORB: one pyramid level (ORB::compute describes provided keypoints on level 0 only), no divisibility requirement
+static int gftt_geometry(lcd_engine * e, int width, int height, const lcd_orb_params * p, OrbGeom & g)
+{
+	if (!p) LCD_FAIL(e, LCD_ERR_INVALID, "null ORB parameters");
+	if (p->patch_size != 31) LCD_FAIL(e, LCD_ERR_INVALID, "only ORB/PatchSize=31 is implemented");
+	if (width < 8 || height < 8) LCD_FAIL(e, LCD_ERR_INVALID, "image must be at least 8x8");
+	if (static_cast<long long>(width) * height >= (1 << 24)) LCD_FAIL(e, LCD_ERR_CAPACITY, "image too large");
+	if (p->n_features <= 0) LCD_FAIL(e, LCD_ERR_INVALID, "Kp/MaxFeatures must be positive");
+	if (p->edge_threshold < 0) LCD_FAIL(e, LCD_ERR_INVALID, "ORB/EdgeThreshold must be >= 0");
+	g.n_levels = 1;
+	g.w[0] = width;
+	g.h[0] = height;
+	g.off[0] = 0;
+	g.frame_stride = width * height;
+	g.n_per_level[0] = p->n_features;
+	g.edge = p->edge_threshold;
+	g.fast_thr = p->fast_threshold;
+	g.patch = p->patch_size;
+	return LCD_OK;
+}
+
+// the host entry points' report of a truncated candidate list (o_overflow)
+static int detect_overflow(lcd_engine * e)
+{
+	if (e->detector == LCD_DETECTOR_GFTT_ORB)
+		LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d GFTT candidate corners in a frame: raise GFTT/QualityLevel", kGfttCandCap);
+	LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d FAST corners in pyramid level 0 (half as many per further level): raise FAST/Threshold", kOrbCandCap);
+}
+
+// GFTT corners of frames [frame0, frame0 + n_frames) straight into the keypoint rows (d_kp / d_n already offset to frame0):
+// eigenvalue stencil, candidates, selection + ORB::compute's border filter.
+static int gftt_detect(lcd_engine * e, int n_frames, int frame0, int total_frames, const OrbGeom & g, const uint8_t * w_gray, const uint8_t * w_mask,
+                       int max_corners, int cap, OrbKeypoint * d_kp, int * d_n, cudaStream_t s)
+{
+	const lcd_gftt_params & gp = e->gftt;
+	const int w = g.w[0], h = g.h[0];
+	const size_t px = static_cast<size_t>(w) * h;
+	const int wpr = (w + 31) / 32;
+	LCD_CUDA(e, e->g_eig.reserve(static_cast<size_t>(total_frames) * px, 0, false, s));
+	LCD_CUDA(e, e->g_max.reserve(total_frames, 0, false, s));
+	LCD_CUDA(e, e->g_cand.reserve(static_cast<size_t>(total_frames) * kGfttCandCap, 0, false, s));
+	LCD_CUDA(e, e->g_cand_count.reserve(total_frames, 0, false, s));
+	if (gp.block_size == 7) LCD_CUDA(e, e->g_rowsum.reserve(static_cast<size_t>(total_frames) * px * 3, 0, false, s));
+	// occupancy bitmap of the accepted corners: shared memory beside the sort buffer when it fits
+	const size_t occ_bytes = static_cast<size_t>(h) * wpr * 4;
+	const size_t sort_bytes = static_cast<size_t>(kGfttSortCap) * sizeof(unsigned long long);
+	const bool occ_smem = sort_bytes + occ_bytes <= 200 * 1024;
+	if (!occ_smem) LCD_CUDA(e, e->g_occ.reserve(static_cast<size_t>(total_frames) * h * wpr, 0, false, s));
+	LCD_CUDA(e, zero_fill_async(e->g_max.p + frame0, n_frames * sizeof(uint32_t), s));
+	LCD_CUDA(e, zero_fill_async(e->g_cand_count.p + frame0, n_frames * sizeof(int), s));
+	GfttArgs a{};
+	a.gray = w_gray;
+	a.mask = w_mask;
+	a.w = w;
+	a.h = h;
+	a.frame_stride = g.frame_stride;
+	const double scale = 1.0 / (4.0 * gp.block_size * 255.0);
+	a.k0 = static_cast<float>(scale);
+	a.k1 = static_cast<float>(2.0 * scale);
+	a.eig = e->g_eig.p + static_cast<size_t>(frame0) * px;
+	a.max_bits = e->g_max.p + frame0;
+	a.rowsum = gp.block_size == 7 ? e->g_rowsum.p + static_cast<size_t>(frame0) * px * 3 : nullptr;
+	if (gp.block_size == 7)
+	{
+		gftt_rowsum7_kernel<<<dim3((h + 127) / 128, n_frames), 128, 0, s>>>(a);
+		LCD_CHECK_LAUNCH(e);
+		gftt_colsum7_kernel<<<dim3((w + 127) / 128, n_frames), 128, 0, s>>>(a);
+	}
+	else if (gp.block_size == 5)
+		gftt_eigen_kernel<5><<<dim3((w + 4 * 28 - 1) / (4 * 28), n_frames), 128, 0, s>>>(a);
+	else
+		gftt_eigen_kernel<3><<<dim3((w + 4 * 30 - 1) / (4 * 30), n_frames), 128, 0, s>>>(a);
+	LCD_CHECK_LAUNCH(e);
+	unsigned long long * cand = e->g_cand.p + static_cast<size_t>(frame0) * kGfttCandCap;
+	int * cand_count = e->g_cand_count.p + frame0;
+	gftt_candidate_kernel<<<dim3((w + 31) / 32, (h + 7) / 8, n_frames), dim3(32, 8), 0, s>>>(a, gp.quality_level, cand, cand_count, e->o_overflow.p);
+	LCD_CHECK_LAUNCH(e);
+	GfttSelectArgs sa{};
+	sa.cand = cand;
+	sa.cand_count = cand_count;
+	sa.w = w;
+	sa.h = h;
+	sa.min_distance = gp.min_distance;
+	sa.min_distance2 = gp.min_distance * gp.min_distance;
+	sa.cell = gp.min_distance >= 1 ? static_cast<int>(std::nearbyint(gp.min_distance)) : 0; // cvRound: half to even
+	sa.max_corners = max_corners;
+	sa.edge = g.edge;
+	sa.block_size = gp.block_size;
+	sa.occ_global = occ_smem ? nullptr : e->g_occ.p + static_cast<size_t>(frame0) * h * wpr;
+	sa.kp = d_kp;
+	sa.n_kp = d_n;
+	sa.cap = cap;
+	const size_t smem = sort_bytes + (occ_smem ? occ_bytes : 0);
+	LCD_CUDA(e, cudaFuncSetAttribute(gftt_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+	gftt_select_kernel<<<n_frames, kGfttSelectThreads, smem, s>>>(sa);
+	LCD_CHECK_LAUNCH(e);
+	return LCD_OK;
+}
+
+int lcd_set_detector(lcd_engine * e, int strategy, const lcd_gftt_params * gftt)
+{
+	if (!e) return LCD_ERR_INVALID;
+	if (strategy == LCD_DETECTOR_ORB)
+	{
+		e->detector = strategy;
+		return LCD_OK;
+	}
+	if (strategy != LCD_DETECTOR_GFTT_ORB) LCD_FAIL(e, LCD_ERR_INVALID, "Kp/DetectorStrategy %d is not implemented (2 = ORB, 8 = GFTT/ORB)", strategy);
+	if (!gftt) LCD_FAIL(e, LCD_ERR_INVALID, "GFTT/ORB needs its GFTT parameters");
+	if (!(gftt->quality_level > 0.0) || !std::isfinite(gftt->quality_level)) LCD_FAIL(e, LCD_ERR_INVALID, "GFTT/QualityLevel must be > 0");
+	if (!(gftt->min_distance >= 0.0) || !std::isfinite(gftt->min_distance)) LCD_FAIL(e, LCD_ERR_INVALID, "GFTT/MinDistance must be >= 0");
+	if (gftt->block_size != 3 && gftt->block_size != 5 && gftt->block_size != 7) LCD_FAIL(e, LCD_ERR_INVALID, "GFTT/BlockSize must be 3, 5 or 7");
+	if (gftt->use_harris) LCD_FAIL(e, LCD_ERR_INVALID, "GFTT/UseHarrisDetector=true is not implemented");
+	e->gftt = *gftt;
+	e->detector = strategy;
+	return LCD_OK;
+}
+
 // Detect + describe frames [frame0, frame0 + n_frames) of a batch of total_frames (total_frames = 0: the range is the whole
 // batch).  Every input, workspace and output pointer addresses frame 0 of the batch; ranges are independent, so the host
 // path runs them chunk by chunk while the next chunk's images are still on their way over PCIe.
@@ -2038,8 +2165,9 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
                    int * d_n, cudaStream_t s, int frame0 = 0, int total_frames = 0)
 {
 	if (total_frames <= 0) total_frames = frame0 + n_frames;
+	const bool gftt = e->detector == LCD_DETECTOR_GFTT_ORB;
 	OrbGeom g{};
-	LCD_TRY(orb_geometry(e, width, height, p, g));
+	LCD_TRY(gftt ? gftt_geometry(e, width, height, p, g) : orb_geometry(e, width, height, p, g));
 	if (channels != 1 && channels != 3) LCD_FAIL(e, LCD_ERR_INVALID, "images must be 8UC1 or 8UC3 (BGR)");
 	if (cap <= 0 || cap > kMaxFrameQueries) LCD_FAIL(e, LCD_ERR_CAPACITY, "cap must be 1..%d", kMaxFrameQueries);
 	if (!d_depth) depth_type = LCD_DEPTH_NONE;
@@ -2052,10 +2180,13 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
 	const int slots = n_frames * g.n_levels, total_slots = total_frames * g.n_levels, slot0 = frame0 * g.n_levels;
 	int level_cap = 0;
 	for (int l = 0; l < g.n_levels; ++l) level_cap = std::max(level_cap, g.n_per_level[l] + 256);
-	LCD_CUDA(e, e->o_cand.reserve(static_cast<size_t>(total_slots) * kOrbCandCap, 0, false, s));
-	LCD_CUDA(e, e->o_cand_count.reserve(total_slots, 0, false, s));
-	LCD_CUDA(e, e->o_level_n.reserve(total_slots, 0, false, s));
-	LCD_CUDA(e, e->o_level_kp.reserve(static_cast<size_t>(total_slots) * level_cap, 0, false, s));
+	if (!gftt)
+	{
+		LCD_CUDA(e, e->o_cand.reserve(static_cast<size_t>(total_slots) * kOrbCandCap, 0, false, s));
+		LCD_CUDA(e, e->o_cand_count.reserve(total_slots, 0, false, s));
+		LCD_CUDA(e, e->o_level_n.reserve(total_slots, 0, false, s));
+		LCD_CUDA(e, e->o_level_kp.reserve(static_cast<size_t>(total_slots) * level_cap, 0, false, s));
+	}
 	if (frame0 == 0)
 	{
 		// the "candidate list truncated" flag of this batch: cleared here, read back by the host entry points
@@ -2079,10 +2210,10 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
 	uint8_t * const w_gray = e->o_gray.p + static_cast<size_t>(frame0) * g.frame_stride;
 	uint8_t * const w_blur = e->o_blur.p + static_cast<size_t>(frame0) * g.frame_stride;
 	uint8_t * const w_mask = use_mask ? e->o_mask.p + static_cast<size_t>(frame0) * g.frame_stride : nullptr;
-	uint32_t * const w_cand = e->o_cand.p + static_cast<size_t>(slot0) * kOrbCandCap;
-	int * const w_cand_count = e->o_cand_count.p + slot0;
-	int * const w_level_n = e->o_level_n.p + slot0;
-	OrbKeypoint * const w_level_kp = e->o_level_kp.p + static_cast<size_t>(slot0) * level_cap;
+	uint32_t * const w_cand = gftt ? nullptr : e->o_cand.p + static_cast<size_t>(slot0) * kOrbCandCap;
+	int * const w_cand_count = gftt ? nullptr : e->o_cand_count.p + slot0;
+	int * const w_level_n = gftt ? nullptr : e->o_level_n.p + slot0;
+	OrbKeypoint * const w_level_kp = gftt ? nullptr : e->o_level_kp.p + static_cast<size_t>(slot0) * level_cap;
 	d_kp += static_cast<size_t>(frame0) * cap;
 	d_n += frame0;
 	if (d_desc) d_desc += static_cast<size_t>(frame0) * cap * 32;
@@ -2104,7 +2235,7 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
 		e->gauss_sigma_loaded = 2.0f;
 	}
 	prof_mark(e, LCD_PROF_ORB, s);
-	LCD_CUDA(e, zero_fill_async(w_cand_count, slots * sizeof(int), s));
+	if (!gftt) LCD_CUDA(e, zero_fill_async(w_cand_count, slots * sizeof(int), s));
 	{
 		OrbPrepArgs a{};
 		a.images = d_images;
@@ -2178,6 +2309,9 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
 		}
 		LCD_CUDA(e, cudaEventRecord(e->aux_blur_done, bs));
 	}
+	if (gftt)
+		LCD_TRY(gftt_detect(e, n_frames, frame0, total_frames, g, w_gray, w_mask, p->n_features, cap, d_kp, d_n, s));
+	else
 	{
 		OrbSelectArgs a{};
 		a.gray = w_gray;
@@ -2221,8 +2355,6 @@ static int orb_run(lcd_engine * e, int n_frames, const uint8_t * d_images, int w
 			if (l > 0 && l <= 3) LCD_CUDA(e, cudaEventRecord(e->aux_join[l - 1], ls));
 		}
 		for (int l = 1; l < g.n_levels && l <= 3; ++l) LCD_CUDA(e, cudaStreamWaitEvent(s, e->aux_join[l - 1], 0));
-	}
-	{
 		int pad = 1;
 		while (pad < g.n_levels * level_cap) pad <<= 1;
 		orb_merge_kernel<<<n_frames, 1024, pad * sizeof(unsigned long long), s>>>(w_level_kp, w_level_n, g.n_levels, level_cap, p->n_features,
@@ -2322,7 +2454,7 @@ int lcd_orb_detect_describe(lcd_engine * e, int n_frames, const uint8_t * images
 	int overflow = 0;
 	LCD_CUDA(e, cudaMemcpyAsync(&overflow, e->o_overflow.p, sizeof(int), cudaMemcpyDeviceToHost, s));
 	LCD_CUDA(e, cudaStreamSynchronize(s));
-	if (overflow) LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d FAST corners in pyramid level 0 (half as many per further level): raise FAST/Threshold", kOrbCandCap);
+	if (overflow) return detect_overflow(e);
 	return LCD_OK;
 }
 
@@ -2356,6 +2488,7 @@ long long lcd_debug_orb_buffer(lcd_engine * e, int which, void * out, long long 
 	case 3: src = e->o_cand.p; bytes = e->o_cand.cap * sizeof(uint32_t); break;
 	case 4: src = e->o_cand_count.p; bytes = e->o_cand_count.cap * sizeof(int); break;
 	case 5: src = e->o_level_n.p; bytes = e->o_level_n.cap * sizeof(int); break;
+	case 10: src = e->g_eig.p; bytes = e->g_eig.cap * sizeof(float); break;
 	case 7: src = e->v_clk.p; bytes = e->v_clk.cap * sizeof(long long); break;
 #ifdef LCD_DEBUG_PHASES
 	case 9:
@@ -3158,8 +3291,7 @@ int lcd_process_frames(lcd_engine * e, int n_frames, const uint8_t * images, int
 	LCD_CUDA(e, cudaMemcpyAsync(e->h_overflow.p, e->o_overflow.p, sizeof(int), cudaMemcpyDeviceToHost, s));
 	if (vp && results) LCD_TRY(verify_download(e, n_frames, 0, results, nullptr, nullptr, s));
 	LCD_CUDA(e, cudaStreamSynchronize(s));
-	if (*e->h_overflow.p)
-		LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d FAST corners in pyramid level 0 (half as many per further level): raise FAST/Threshold", kOrbCandCap);
+	if (*e->h_overflow.p) return detect_overflow(e);
 	return LCD_OK;
 }
 
@@ -3273,8 +3405,7 @@ int lcd_process_frames_wait(lcd_engine * e)
 	f.user_results = nullptr;
 	e->flight_head ^= 1;
 	--e->flights_busy;
-	if (f.overflow.p && *f.overflow.p)
-		LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d FAST corners in pyramid level 0 (half as many per further level): raise FAST/Threshold", kOrbCandCap);
+	if (f.overflow.p && *f.overflow.p) return detect_overflow(e);
 	return LCD_OK;
 }
 
@@ -3537,8 +3668,7 @@ int lcd_map_frame(lcd_engine * e, int sig_id, int incremental, float nndr, int n
 	--e->map_busy;
 	ms.busy = false;
 	if (rc != LCD_OK) return rc;
-	if (*ms.h_overflow.p)
-		LCD_FAIL(e, LCD_ERR_CAPACITY, "more than %d FAST corners in pyramid level 0 (half as many per further level): raise FAST/Threshold", kOrbCandCap);
+	if (*ms.h_overflow.p) return detect_overflow(e);
 	if (n_kp_out) *n_kp_out = n_kp;
 	if (n_new_out) *n_new_out = n_new;
 	if (kp_out) LCD_CUDA(e, cudaMemcpyAsync(kp_out, ms.kp.p, static_cast<size_t>(n_kp) * sizeof(OrbKeypoint), cudaMemcpyDeviceToHost, s));

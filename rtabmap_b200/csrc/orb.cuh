@@ -106,6 +106,7 @@ __global__ void orb_prepare_kernel(const OrbPrepArgs a)
 		for (int dx = 0; dx < 2; ++dx)
 		{
 			const int x = 2 * x1 + dx, y = 2 * y1 + dy;
+			if (x >= w || y >= h) continue; // odd sizes (one pyramid level only)
 			int gv;
 			if (a.channels == 1) gv = img[static_cast<size_t>(y) * w + x];
 			else
